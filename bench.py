@@ -15,6 +15,10 @@ e2e    = same, through the public petit_kernel Python API with the activations c
 roofline / cpu_baseline / clocks / details: see DESIGN.md "Measurement".
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--m M]
+                  [--dump-outputs DIR]
+
+--dump-outputs DIR writes the outputs of the last timed step as DIR/<gemm>.npy (float32) so
+that two builds can be compared output for output: the inputs depend only on the arguments.
 """
 from __future__ import annotations
 
@@ -35,6 +39,25 @@ sys.path.insert(0, ROOT)
 LAYER = [("qkv", 10240, 8192, "column"), ("o", 8192, 8192, "row"),
          ("gate_up", 57344, 8192, "column"), ("down", 8192, 28672, "row")]
 METRIC = "FP4xBF16 GEMM algorithmic HBM GB/s, Llama-3.3-70B decoder-layer GEMM set (NVFP4, M=16)"
+DUMP_LIMIT = 64 << 20  # bytes written by --dump-outputs, per run
+
+
+def dump_outputs(dirname, named, limit=DUMP_LIMIT, suffix=""):
+    """Write each [m, n] output of `named` ((name, tensor) pairs) as DIR/<name><suffix>.npy in
+    float32.  Above `limit` bytes in all, the same seeded sample of rows is kept from each."""
+    import numpy as np
+
+    os.makedirs(dirname, exist_ok=True)
+    m = named[0][1].shape[0]
+    row_bytes = sum(c[0].numel() for _, c in named) * 4
+    rows = None
+    if m * row_bytes > limit:
+        keep = max(1, limit // row_bytes)
+        rows = torch.from_numpy(np.sort(np.random.RandomState(0).choice(m, keep, replace=False)))
+    for name, c in named:
+        if rows is not None:
+            c = c[rows.to(c.device)]
+        np.save(os.path.join(dirname, name + suffix + ".npy"), c.float().cpu().numpy())
 
 
 def algo_bytes(m, n, k, group=16):
@@ -101,25 +124,31 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------ CPU reference arm
+def cpu_case(g, m, n, k):
+    """One seeded NVFP4 problem for the CPU arm: activations, packed weights, scales, global scale."""
+    a = torch.randn((m, k), generator=g).to(torch.bfloat16)
+    q = torch.randint(0, 256, (n, k // 2), generator=g, dtype=torch.uint8)
+    s = (torch.rand((n, k // 16), generator=g) * 3.5 + 0.25).to(torch.float8_e4m3fn)
+    return a, q, s, torch.ones(1)
+
+
 def cpu_reference_rate(m, shapes, reps):
     """The reference's CPU path (torch dequantise + fp32 matmul,
     tests/ops/test_fp4_gemm_quark.py:9-24) restated in oracle/, on the host cores."""
     from oracle import petit_oracle as orc
 
     g = torch.Generator().manual_seed(0)
-    total_bytes, total_s = 0, 0.0
-    for (_, n, k, _) in shapes:
-        a = torch.randn((m, k), generator=g).to(torch.bfloat16)
-        q = torch.randint(0, 256, (n, k // 2), generator=g, dtype=torch.uint8)
-        s = (torch.rand((n, k // 16), generator=g) * 3.5 + 0.25).to(torch.float8_e4m3fn)
-        gs = torch.ones(1)
+    total_bytes, total_s, last = 0, 0.0, []
+    for (nm, n, k, _) in shapes:
+        a, q, s, gs = cpu_case(g, m, n, k)
         orc.nvfp4_gemm_ref_torch(a[:, :256], q[:64, :128], s[:64, :16], gs)  # warm torch
         t0 = time.perf_counter()
         for _ in range(reps):
-            orc.nvfp4_gemm_ref_torch(a, q, s, gs)
+            c = orc.nvfp4_gemm_ref_torch(a, q, s, gs)
         total_s += time.perf_counter() - t0
         total_bytes += reps * algo_bytes(m, n, k)
-    return total_bytes / total_s / 1e9, total_s
+        last.append((nm, c))
+    return total_bytes / total_s / 1e9, total_s, last
 
 
 def run_reference(args):
@@ -130,12 +159,14 @@ def run_reference(args):
     # every N, so its value does not depend on how it was launched
     torch.set_num_threads(os.cpu_count() or 1)
     shapes = [LAYER[1]]  # o_proj 8192 x 8192: bounded sample of the layer set
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     for _ in range(min(args.warmup, 1)):
         cpu_reference_rate(args.m, shapes, 1)
     t0 = time.perf_counter()
-    gbs, secs = cpu_reference_rate(args.m, shapes, steps)
+    gbs, secs, last = cpu_reference_rate(args.m, shapes, steps)
     wall = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     out = {
         "impl": "reference", "metric": METRIC, "value": gbs, "unit": "GB/s",
         "n_gpus": args.gpus, "steps": steps, "warmup": min(args.warmup, 1),
@@ -163,10 +194,37 @@ def workload_config(args, world):
 
 
 # ------------------------------------------------------------------ GPU arm
+def make_inputs(pk, shard, m, dev, rank):
+    """Seeded inputs of the GPU arm: `copies` distinct packed copies of the (sharded) layer set,
+    together larger than L2, the global scale and one activation per K.  The same arguments
+    always give the same inputs.  Returns them with the generator, which later code draws on."""
+    set_bytes = sum(n * k // 2 + n * k // 16 for _, n, k, _ in shard)
+    copies = max(2, int(300e6 // set_bytes) + 2)
+    g = torch.Generator(device=dev).manual_seed(1234 + rank)
+    layers = []
+    for _ in range(copies):
+        one = []
+        for nm, n, k, kind in shard:
+            q = torch.randint(0, 256, (n, k // 2), generator=g, dtype=torch.uint8, device=dev)
+            s = (torch.rand((n, k // 16), generator=g, device=dev) * 3.5 + 0.25).to(torch.float8_e4m3fn)
+            b = pk.repack_nvfp4(q.view(torch.int32), n, k)
+            sp = pk.process_nvfp4_scales(s, n, k)
+            one.append((nm, n, k, kind, b, sp))
+            del q, s
+        layers.append(one)
+    gs = torch.rand(1, generator=g, device=dev) * 1.5 + 0.5
+    acts = {k: torch.randn((m, k), generator=g, device=dev, dtype=torch.float32).to(torch.bfloat16)
+            for k in {k for _, _, k, _ in shard}}
+    return layers, copies, gs, acts, g
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=500)
+    ap.add_argument("--steps", type=int, default=500,
+                    help="timed steps.  With --impl reference every step is a host-CPU pass of the "
+                         "o_proj dequantise + fp32 matmul (about 0.3 s on an 8-core x86 host), so "
+                         "the default of 500 takes minutes there")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--m", type=int, default=16)
@@ -175,7 +233,13 @@ def main():
                     help="skip the cuBLAS / vLLM Marlin comparator rows of `details`")
     ap.add_argument("--graph", action="store_true",
                     help="replay one captured CUDA graph per layer step instead of eager launches")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<gemm>.npy (float32; "
+                         "a seeded sample of rows when they exceed 64 MB; one file per rank "
+                         "with --gpus > 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -198,23 +262,7 @@ def main():
 
     # ---- build the (sharded) layer set, several distinct copies to defeat L2
     shard = [(nm,) + petit_tp.shard_shape(n, k, kind, world) + (kind,) for nm, n, k, kind in LAYER]
-    set_bytes = sum(n * k // 2 + n * k // 16 for _, n, k, _ in shard)
-    copies = max(2, int(300e6 // set_bytes) + 2)
-    g = torch.Generator(device=dev).manual_seed(1234 + rank)
-    layers = []
-    for _ in range(copies):
-        one = []
-        for nm, n, k, kind in shard:
-            q = torch.randint(0, 256, (n, k // 2), generator=g, dtype=torch.uint8, device=dev)
-            s = (torch.rand((n, k // 16), generator=g, device=dev) * 3.5 + 0.25).to(torch.float8_e4m3fn)
-            b = pk.repack_nvfp4(q.view(torch.int32), n, k)
-            sp = pk.process_nvfp4_scales(s, n, k)
-            one.append((nm, n, k, kind, b, sp))
-            del q, s
-        layers.append(one)
-    gs = torch.rand(1, generator=g, device=dev) * 1.5 + 0.5
-    acts = {k: torch.randn((m, k), generator=g, device=dev, dtype=torch.float32).to(torch.bfloat16)
-            for k in {k for _, _, k, _ in shard}}
+    layers, copies, gs, acts, g = make_inputs(pk, shard, m, dev, rank)
 
     # row-parallel outputs (o, down): PETIT_TP_ALLREDUCE = fused (default) | peer | nccl | symm
     #   fused: ONE kernel per rank computes the K-split GEMM and all-reduces its output -- the
@@ -329,6 +377,7 @@ def main():
     # and capturing NCCL collectives hung at TP2 on this stack.
     use_graph = args.graph
     graphs = None
+    graph_outs = []
     if use_graph:
         try:
             for i in range(copies):  # warm every path (workspace, NCCL) before capture
@@ -339,7 +388,7 @@ def main():
             for i in range(copies):
                 gph = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(gph, stream=side):
-                    layer_step(i)
+                    graph_outs.append(layer_step(i))
                 graphs.append(gph)
             sync()
         except Exception as exc:
@@ -352,8 +401,8 @@ def main():
     def timed_step(i):
         if graphs is not None:
             graphs[i % copies].replay()
-        else:
-            eager_step(i)
+            return graph_outs[i % copies]
+        return eager_step(i)
 
     # ---- device-resident timing
     for i in range(args.warmup):
@@ -365,8 +414,11 @@ def main():
     sync()
     lo = sampler.mark()
     e0.record()
-    for i in range(args.steps):
+    for i in range(args.steps - 1):
         timed_step(i)
+    # only the last step's outputs are kept (--dump-outputs): every earlier step drops its
+    # own before the next allocates, so the allocator hands out the same blocks each step
+    last = timed_step(args.steps - 1)
     e1.record()
     sync()
     ms = e0.elapsed_time(e1)
@@ -384,6 +436,11 @@ def main():
     clocks = sampler.stop(lo, hi) if rank == 0 else None
     if clocks is not None:
         clocks["window"] = "timed region" if hi - lo >= 3 else "timed region + same load repeated"
+    if args.dump_outputs:
+        # (the untimed filler load above allocates its own outputs: `last` is untouched)
+        dump_outputs(args.dump_outputs, [(x[0], c) for x, c in zip(shard, last)],
+                     DUMP_LIMIT // world, f"_rank{rank}" if world > 1 else "")
+    del last
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -590,7 +647,7 @@ def main():
     torch.set_num_threads(os.cpu_count() or 1)  # torchrun pins OMP_NUM_THREADS=1
     cores = torch.get_num_threads()
     t0 = time.perf_counter()
-    cpu_gbs, cpu_s = cpu_reference_rate(m, [LAYER[1]], 2)
+    cpu_gbs, cpu_s, _ = cpu_reference_rate(m, [LAYER[1]], 2)
     cpu = {"value": round(cpu_gbs, 3), "unit": "GB/s", "cores": cores, "kind": "port",
            "sample": f"o_proj 8192x8192 NVFP4 M={m}, 2 passes of the torch dequant+fp32-matmul "
                      f"oracle on the host ({time.perf_counter() - t0:.1f} s)"}
