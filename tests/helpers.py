@@ -57,3 +57,14 @@ def pack_mxfp4(pk, q_u8, scales, n, k):
     b = pk.repack_mxfp4(q_u8.cuda().contiguous().view(torch.int32), n, k)
     s = pk.process_mxfp4_scales(scales.cuda(), n, k)
     return b, s
+
+
+def stream_k_cuts_fn(lib):
+    """cuts_fn for oracle.stream_k_plan: the launcher's range cuts (petit_debug_stream_k_cuts)."""
+
+    def cuts(units, k_tiles, grid, lat, late):
+        out = (ctypes.c_uint * (grid + 1))()
+        assert lib.petit_debug_stream_k_cuts(units, k_tiles, grid, lat, late, out) == 0
+        return list(out)
+
+    return cuts

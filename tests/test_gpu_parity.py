@@ -185,6 +185,13 @@ def run_gemm_case(pk, fmt, dtype, m, n, k, solution_id=-1, seed=42):
     ref = gpu_ref_f32(pk, a.cuda(), b, sp, gs, n, k, mx)
     err = orc.max_rel_err(c, ref)
     assert err <= GEMM_TOL, f"{fmt} {dtype} m={m} n={n} k={k} sol={solution_id}: max rel err {err}"
+    # per element, against the oracle's own dequantisation (sampled rows of large weights)
+    rows = np.arange(n) if n * k <= 1 << 26 else np.unique(np.concatenate(
+        [np.arange(128), np.arange(n - 128, n), np.random.RandomState(0).choice(n, 256, replace=False)]))
+    sb = s.numpy() if mx else s.view(torch.uint8).numpy()
+    w = (orc.dequant_mxfp4 if mx else orc.dequant_nvfp4)(q.numpy()[rows], sb[rows])
+    assert orc.elementwise_ok(c[:, torch.from_numpy(rows).cuda()], a.cuda(), w, gs.item(), dtype), \
+        f"{fmt} {dtype} m={m} n={n} k={k} sol={solution_id}: elementwise"
     return c
 
 
@@ -489,8 +496,10 @@ def test_prefill_tiles_and_cluster_variant(pk, m, n, k):
     outs = [pk.mul_nvfp4_a16(ac, b, sp, gsc, m, n, k, -1)]
     for sid in sols:
         outs.append(pk.mul_nvfp4_a16(ac, b, sp, gsc, m, n, k, int(sid)))
+    w = orc.dequant_nvfp4(q.numpy(), s.view(torch.uint8).numpy())
     for o in outs:
         assert orc.max_rel_err(o.float().cpu(), want) <= GEMM_TOL
+        assert orc.elementwise_ok(o, ac, w, gs.item(), torch.bfloat16)
     # every tile shape computes the same sums up to fp32 accumulation order
     for o in outs[1:]:
         assert orc.max_rel_err(o.float().cpu(), outs[0].float().cpu()) <= GEMM_TOL
@@ -538,10 +547,12 @@ def test_fused_bias_and_residual_epilogue(pk, fmt, dtype, m, n, k):
                                         None if bb is None else bb.cuda(),
                                         None if rr is None else rr.cuda())
         assert got.dtype == dtype and orc.max_rel_err(got, want) <= GEMM_TOL
+        assert orc.elementwise_ok(got, ac, w, gs.item(), dtype, bb, rr)
     # residual may alias the output (in-place residual stream update)
     out = resid.cuda().clone()
     pk.ops.mul_fp4_a16_ex_out(out, ac, b, sp, gsc, m, n, k, -1, mx, bias.cuda(), out)
     assert orc.max_rel_err(out, ref32 + bias.float() + resid.float()) <= GEMM_TOL
+    assert orc.elementwise_ok(out, ac, w, gs.item(), dtype, bias, resid)
     # the glue uses it instead of output.add_(bias)
     from petit_kernel import petit_utils as pu
 
@@ -609,7 +620,7 @@ def test_grouped_moe_gemm(pk, fmt):
         total = offsets[-1]
         if fmt == "mxfp4":
             n = (n + 31) // 32 * 32
-        a_all, bs, ss, gss, refs = [], [], [], [], []
+        a_all, bs, ss, gss, refs, ws = [], [], [], [], [], []
         for g in range(e):
             a, q, s, gs = make(max(counts[g], 1), n, k, 100 + g)
             a = a[:counts[g]]
@@ -621,6 +632,7 @@ def test_grouped_moe_gemm(pk, fmt):
             else:  # many experts: reuse the 8th expert's weights, own activations and scale
                 b, sp = bs[7], ss[7]
             refs.append((a.float() @ wt) * gs.item())
+            ws.append(w)
             a_all.append(a); bs.append(b); ss.append(sp); gss.append(gs)
         a_cat = torch.cat(a_all).cuda().contiguous()
         outs = []
@@ -640,6 +652,9 @@ def test_grouped_moe_gemm(pk, fmt):
         for g in range(e):
             if counts[g]:
                 assert orc.max_rel_err(outs[0][offsets[g]:offsets[g + 1]].cpu(), refs[g]) <= GEMM_TOL
+                for o in outs:
+                    assert orc.elementwise_ok(o[offsets[g]:offsets[g + 1]], a_all[g].cuda(), ws[g],
+                                              gss[g].item(), torch.bfloat16), (n, k, counts, g)
         assert pk.ops.workspace_status() == 0
 
 
