@@ -225,8 +225,8 @@ int petit_allreduce_oneshot(void *out, const void *const *peer_bufs, void *const
  * Every rank calls it for every GEMM of the group, in the same order, with the same m <= 64,
  * n and solution id (the call is CUDA-graph capturable; the call counter lives in `state`).
  * A peer that does not deliver within PETIT_WATCHDOG_MS makes the waiting CTA go on without
- * it; petit_fused_allreduce_status (synchronises the stream) then returns 1 + that rank,
- * else 0 (-1: CUDA error). */
+ * it; petit_fused_allreduce_status (synchronises the stream) then returns 1 (it does not say
+ * which peer was missing), else 0 (-1: CUDA error). */
 typedef struct PetitFusedAllReduce {
     int32_t world, rank;
     void *recv[8];

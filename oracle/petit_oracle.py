@@ -446,8 +446,8 @@ def ring_fit(mode: str, ntok: int) -> int:
 
 def stream_k_plan(m: int, n: int, k: int, ntok: int, num_sms: int, pdl: bool, cluster: bool,
                   cuts_fn, mode: str = "nv_bf16", whole_tiles_rule: bool = True,
-                  tilt_units: int = -1, tilt_late: int = -1):
-    """Grid, range cuts and per-tile reducer facts of one (non-grouped, non-all-reduce) launch.
+                  tilt_units: int = -1, tilt_late: int = -1, all_reduce: bool = False):
+    """Grid, range cuts and per-tile reducer facts of one (non-grouped) launch.
 
     cuts_fn(units, k_tiles, grid, lat, late) -> grid + 1 cuts: the library's
     petit_debug_stream_k_cuts (lat = late = 0 gives the equal split).  `cluster` is the
@@ -455,7 +455,14 @@ def stream_k_plan(m: int, n: int, k: int, ntok: int, num_sms: int, pdl: bool, cl
     PETIT_TILT_UNITS / PETIT_TILT_LATE (-1: unset).  Each tile entry: contributors (CTAs other
     than the reducer that add a partial; 0 = unsplit), m_valid, n_partial, and the reducer path
     of its first 16 tokens ('reg' <= 3 contributors, 'ring' up to ring_fit, else 'reg' over all
-    of them) and whether tokens 16.. reach the L2 tail loop."""
+    of them) and whether tokens 16.. reach the L2 tail loop.
+
+    all_reduce: the GEMM fused with its all-reduce (launch_mode with ar_world > 1, i.e.
+    launch_variant<..., CL = false, AR = true>): decode tiles only (ntok 16 / 32 / 64, m <= 64),
+    never a cluster, and no arrival term in the cut tilt (late = 0)."""
+    if all_reduce:
+        assert ntok in (16, 32, 64) and 1 <= m <= 64, (ntok, m)
+        cluster = False
     num_sms = min(num_sms, MAX_GRID)
     n_tiles = (n + TILE_N - 1) // TILE_N
     m_tiles = (m + ntok - 1) // ntok
@@ -476,7 +483,7 @@ def stream_k_plan(m: int, n: int, k: int, ntok: int, num_sms: int, pdl: bool, cl
     lat = late = 0
     if tilt:
         lat = tilt_units if tilt_units >= 0 else (5 if ntok <= 32 else 3)
-        late = 0 if not pdl else (tilt_late if tilt_late >= 0 else (4 if ntok <= 32 else 3))
+        late = 0 if (not pdl or all_reduce) else (tilt_late if tilt_late >= 0 else (4 if ntok <= 32 else 3))
     cuts = list(cuts_fn(units, k_tiles, sched_grid, lat, late))
     assert cuts[0] == 0 and cuts[-1] == units and len(cuts) == sched_grid + 1
 
@@ -530,3 +537,17 @@ def plan_paths(plan) -> set:
         if t["m_valid"] < plan["ntok"]:
             got.add("split_partial_m")
     return got
+
+
+def rank_order_sum(partials, dtype) -> torch.Tensor:
+    """What the fused all-reduce computes from the ranks' 16-bit partial outputs (one-shot and
+    two-shot alike): an fp32 sum that starts from +0.0f and adds ranks 0 .. world - 1 in that
+    order, each addition rounded to fp32, then one RN16.  partials: 16-bit tensors of one
+    shape, rank 0 first."""
+    dt = _torch_dtype(dtype)
+    acc = np.zeros(tuple(partials[0].shape), dtype=np.float32)
+    with np.errstate(over="ignore", invalid="ignore"):
+        for p in partials:
+            assert p.dtype == dt, (p.dtype, dt)
+            acc = (acc + p.detach().cpu().float().numpy()).astype(np.float32)
+    return rn16(acc, dt)

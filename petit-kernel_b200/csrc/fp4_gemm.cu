@@ -1121,6 +1121,11 @@ fp4_gemm_kernel(const __grid_constant__ CUtensorMap tmap_act,
                     //    over all the CTAs that finish tiles.
                     // Two buffer parities alternate per call: a rank can only get one call ahead
                     // of a peer (it needs that peer's packets to finish a call).
+                    // Epoch 0 is never used: a slot no call has written yet is all zero bytes,
+                    // i.e. a valid packet of epoch 0 holding 0, which a reader would take for a
+                    // peer's partial.  So the call counter state[0] runs modulo kArCallPeriod =
+                    // 2^32 - 2 and the epochs run 1 .. 2^32 - 2; the period is even, so the
+                    // parity still alternates from one call to the next across the wrap.
                     const uint32_t epoch = ar_epoch + 1;
                     const uint32_t n_slots = sched_tiles_n * (kArMaxTokens / 16);
                     const uint32_t slot = g.n_tile * (kArMaxTokens / 16) + (m0 + (uint32_t)c0) / 16;
@@ -1383,13 +1388,15 @@ fp4_gemm_kernel(const __grid_constant__ CUtensorMap tmap_act,
         __syncthreads();
     if (threadIdx.x == 0) trace_stamp(args, 8);
     if (warp == kMmaWarp) tmem_dealloc(tmem, 512);
-    // fused all-reduce: the last CTA to exit advances the call epoch (every CTA read it at its
-    // start; the next launch reads it after this grid has completed)
+    // fused all-reduce: the last CTA to exit advances the call counter (every CTA read it at its
+    // start; the next launch reads it after this grid has completed), modulo kArCallPeriod so
+    // that the epoch (counter + 1) is never 0 -- see the packet format above
     if (AR && threadIdx.x == 0) {
         __threadfence();
         if (atomicAdd(args.ar_state + 1, 1u) == gridDim.x - 1) {
             args.ar_state[1] = 0;
-            args.ar_state[0] += 1;
+            const uint32_t next = args.ar_state[0] + 1;
+            args.ar_state[0] = next == kArCallPeriod ? 0u : next;
         }
     }
 }

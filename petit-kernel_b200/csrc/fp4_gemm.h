@@ -44,9 +44,11 @@ struct GemmArgs {
     // buffer as self-validating {data, epoch} packets and sums the peers' packets of the same
     // tile in rank order before it stores the tile (see fp4_gemm.cu, "fused all-reduce").
     uint32_t ar_world, ar_rank;
-    uint32_t ar_two_shot;      // 0: every rank sums every tile; 1: tile t is reduced by rank t % world
+    uint32_t ar_two_shot;      // 0: every rank sums every row; 1: row r of a tile is reduced by
+                               //    rank r / (128 / world)
     uint8_t *ar_recv[8];       // rank p's receive buffer as mapped in this process
-    unsigned *ar_state;        // local device words: [0] epoch, [1] exited-CTA counter, [2] status
+    unsigned *ar_state;        // local device words: [0] call counter (epoch - 1), [1] exited-CTA
+                               // counter, [2] status
 };
 
 // Receive-buffer geometry of the fused all-reduce: [parity 2][source rank 8][slot][8 KB], one slot
@@ -54,6 +56,8 @@ struct GemmArgs {
 constexpr unsigned kArMaxWorld = 8;
 constexpr unsigned kArMaxTokens = 64;
 constexpr unsigned kArSlotBytes = 8192;
+// The call counter ar_state[0] wraps at this (even) period, so the epoch is never 0.
+constexpr unsigned kArCallPeriod = 0xFFFFFFFEu;
 inline size_t ar_recv_bytes(unsigned n) {
     return (size_t)2 * kArMaxWorld * ((n + 127) / 128) * (kArMaxTokens / 16) * kArSlotBytes;
 }

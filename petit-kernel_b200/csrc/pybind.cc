@@ -537,15 +537,19 @@ PYBIND11_MODULE(ops, m) {
             hints.b_type = mx ? PETIT_DTYPE_MXFP4_E2M1 : PETIT_DTYPE_FP4_E2M1;
             hints.c_type = a_type;
             hints.require_high_precision = 0;
+            PetitEpilogue epi = {nullptr, nullptr, PETIT_ACT_NONE,
+                                 mx ? PETIT_WEIGHT_LAYOUT_DEFAULT : weight_layout_of(b, sn, sk)};
+            TORCH_CHECK(epi.weight_layout == PETIT_WEIGHT_LAYOUT_DEFAULT || a_type == PETIT_DTYPE_FP16,
+                        "b was repacked for float16 activations; a is bfloat16");
             PetitFusedAllReduce ar;
             ar.world = (int32_t)recv_ptrs.size();
             ar.rank = (int32_t)rank;
             for (int r = 0; r < 8; ++r)
                 ar.recv[r] = r < ar.world ? reinterpret_cast<void *>(recv_ptrs[r]) : nullptr;
             ar.state = state.data_ptr();
-            auto fn = mx ? petit_gemm_mxfp4_a16_allreduce : petit_gemm_nvfp4_a16_allreduce;
+            auto fn = mx ? petit_gemm_mxfp4_a16_ex : petit_gemm_nvfp4_a16_ex;
             int err = fn(c.data_ptr(), a.data_ptr(), b.data_ptr(), s.data_ptr(), gs.data_ptr<float>(),
-                         sm, sn, sk, &hints, static_cast<uint64_t>(sol), &ar, stream_of(a));
+                         sm, sn, sk, &hints, static_cast<uint64_t>(sol), &epi, &ar, stream_of(a));
             check_status(err, sm, sn, sk, sol);
             return c;
         },

@@ -206,3 +206,86 @@ def test_dense_shapes_cover_every_reducer_path(cuts_fn, mode):
     ntoks = {lab: {t for _, t in v} for lab, v in table.items()}
     for lab in ("reg_1_3", "ring", "l2_tail"):
         assert len(ntoks[lab]) >= 2, (lab, ntoks[lab])
+
+
+# ------------------------------------------------------------------ fused all-reduce
+def test_all_reduce_plan_agrees_with_the_launcher(cuts_fn):
+    """launch_mode with ar_world > 1: launch_variant<..., CL = false, AR = true> for 16/32/64-token
+    tiles only (m <= 64), never a cluster, no arrival term in the tilt (late = 0); the grid,
+    whole-tile rule and lat are those of the plain decode launch."""
+    for ntok in (128, 256):
+        with pytest.raises(AssertionError):
+            orc.stream_k_plan(16, 1024, 2048, ntok, 148, True, True, cuts_fn, all_reduce=True)
+    with pytest.raises(AssertionError):
+        orc.stream_k_plan(65, 1024, 2048, 64, 148, True, True, cuts_fn, all_reduce=True)
+    # tilted shape (37 n-tiles x 32 k-tiles): same lat, late 0 even under PDL, so the cuts equal
+    # those of a plain launch without PDL
+    ar = orc.stream_k_plan(16, 37 * 128, 8192, 16, 148, True, True, cuts_fn, all_reduce=True)
+    plain_nopdl = orc.stream_k_plan(16, 37 * 128, 8192, 16, 148, False, True, cuts_fn)
+    plain_pdl = orc.stream_k_plan(16, 37 * 128, 8192, 16, 148, True, True, cuts_fn)
+    assert ar["tilt"] and (ar["lat"], ar["late"]) == (5, 0) and plain_pdl["late"] == 4
+    assert ar["cuts"] == plain_nopdl["cuts"] != plain_pdl["cuts"]
+    # TP-8 o_proj: whole tiles under the all-reduce too; no cluster even where the plain launch has one
+    p = orc.stream_k_plan(16, 8192, 1024, 16, 148, True, True, cuts_fn, all_reduce=True)
+    assert p["whole_tiles"] and p["grid"] == 64 and not p["cluster"]
+    # small shards: one k-tile per CTA, grid = units, contributors = k_tiles - 1
+    p = orc.stream_k_plan(64, 144, 2048, 64, 148, True, True, cuts_fn, all_reduce=True)
+    assert p["grid"] == p["units"] == 16 and [t["contributors"] for t in p["tiles"]] == [7, 7]
+
+
+def test_rank_order_sum_rejects_planted_defects():
+    """rank_order_sum is the fp32 sum from +0.0f in rank order of the 16-bit partials, then RN16.
+    Three planted defects change bits: ranks added in reverse order, the sum formed in fp64, and
+    partials summed before their rounding to 16 bits.  The 1e-2 normwise bar accepts all three;
+    elementwise_ok, with the partials as the inputs of the sum, accepts the first two.  Order-
+    sensitive columns: bf16 (+2^25, +1, -2^25) sums to 0 in rank order and to 1 in fp64;
+    (+2^25, -2^25, +1) to 1 in rank order and to 0 reversed (fp16: 32768 and 2^-10)."""
+    for dt, big, tiny in ((torch.bfloat16, 2.0 ** 25, 1.0), (torch.float16, 32768.0, 2.0 ** -10)):
+        rs = np.random.RandomState(3)
+        raw = (rs.randn(3, 8, 64) * 100).astype(np.float32)   # per-rank fp32 partials, 3 ranks
+        raw[:, :, 0] = np.array([big, tiny, -big], dtype=np.float32)[:, None]
+        raw[:, :, 1] = np.array([big, -big, tiny], dtype=np.float32)[:, None]
+        parts = [torch.from_numpy(x).to(dt) for x in raw]
+        want = orc.rank_order_sum(parts, dt)
+        assert want[:, 0].float().eq(0).all() and want[:, 1].float().eq(tiny).all()
+        f64 = sum(p.double() for p in parts)
+        defects = {
+            "reversed": orc.rank_order_sum(parts[::-1], dt),
+            "fp64_sum": f64.to(dt),
+            "unrounded_partials": orc.rn16(raw.sum(0, dtype=np.float32), dt),
+        }
+        assert defects["reversed"][:, 1].float().eq(0).all() and defects["fp64_sum"][:, 0].float().eq(tiny).all()
+        # the sum as a GEMM: a = the partials side by side, w = three identities
+        a_full = torch.cat([p.double() for p in parts], 1)
+        w = np.hstack([np.eye(64, dtype=np.float32)] * 3)
+        assert orc.elementwise_ok(want, a_full, w, 1.0, dt)
+        for name, c in defects.items():
+            assert not orc.bits_equal_pm0(c, want), (dt, name)
+            assert orc.max_rel_err(c.float(), f64.float()) <= 1e-2, (dt, name)
+            assert orc.elementwise_ok(c, a_full, w, 1.0, dt) == (name != "unrounded_partials"), (dt, name)
+    # the sum starts from +0.0f: -0 + -0 gives +0
+    z = orc.rank_order_sum([torch.tensor([-0.0], dtype=torch.bfloat16)] * 2, torch.bfloat16)
+    assert z.view(torch.int16).item() == 0
+
+
+@pytest.mark.parametrize("mode", list(tge.MODES))
+def test_fused_allreduce_cases_fit_and_cover_every_path(cuts_fn, mode):
+    """Every emulated all-reduce case of tests/test_fused_allreduce_exact.py, at the B200's 148
+    SMs: all ranks' grids fit at once (world x grid, 2 x world x grid for chained calls), every
+    grid is its unit or whole-tile count without tilted cuts, and the calls of the mode reach
+    every reducer path the file requires."""
+    import petit_kernel
+    import test_fused_allreduce_exact as tfa
+
+    for case in tfa.all_cases(petit_kernel, mode):
+        tfa.check_budget(petit_kernel, cuts_fn, mode, case, tfa.AR_SMS)
+    table = tfa.coverage(petit_kernel, cuts_fn, mode)
+    assert [lab for lab in tfa.AR_REQUIRED if lab not in table] == []
+    worlds = {w for w, *_ in tfa.sequence_cases(petit_kernel, mode)}
+    assert worlds == set(range(2, 9))
+    ntoks = {tge.solution_ntok(petit_kernel, mode, 64, n, k, sid) for _, sid, n, k, _ in tfa.sequence_cases(petit_kernel, mode)}
+    assert ntoks == {16, 32, 64}
+    # partial n-tiles of both kinds, and m values that change on every call
+    rems = {n % 128 for _, _, n, _, _ in tfa.sequence_cases(petit_kernel, mode)}
+    assert rems == ({32, 96} if mode in ("mx_bf16", "nv_f16n") else {16, 112})
+    assert all(x != y for x, y in zip(tfa.SEQ_M, tfa.SEQ_M[1:])) and set(tfa.SEQ_M) == {1, 5, 16, 17, 33, 48, 64}

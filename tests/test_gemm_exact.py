@@ -119,12 +119,12 @@ def assert_bits(got, want, what):
         raise AssertionError(f"{what}: {int(bad.sum())} of {bad.numel()} outputs differ, first {idx}: {vals}")
 
 
-def plan_labels(cuts_fn, mode, m, n, k, ntok, sms):
+def plan_labels(cuts_fn, mode, m, n, k, ntok, sms, all_reduce=False):
     """Coverage labels that hold with and without programmatic dependent launch (the first GEMM
     after a repack on a stream runs without it)."""
     got = None
     for pdl in (True, False):
-        p = orc.stream_k_plan(m, n, k, ntok, sms, pdl, True, cuts_fn, mode=mode)
+        p = orc.stream_k_plan(m, n, k, ntok, sms, pdl, True, cuts_fn, mode=mode, all_reduce=all_reduce)
         lab = orc.plan_paths(p)
         got = lab if got is None else got & lab
     return got

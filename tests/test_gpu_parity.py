@@ -782,46 +782,74 @@ def test_bench_matmul_cli_tune(pk):
 
 
 @pytest.mark.parametrize("end_barrier", [True, False])
-def test_peer_allreduce_two_ranks_emulated_on_one_gpu(pk, end_barrier):
-    """csrc/allreduce.cu with world = 2 emulated on one device: both 'ranks' run as
-    concurrent kernels on two streams and exchange flags through each other's pads.
-    Result must be the fp32 sum in rank order, bit-identical on both ranks, for several
-    calls in a row (monotonic flag counters)."""
-    m, n = 16, 2048
+@pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float16])
+@pytest.mark.parametrize("shape", [(16, 2048), (48, 5504)])
+@pytest.mark.parametrize("world", range(2, 9))
+def test_peer_allreduce_two_ranks_emulated_on_one_gpu(pk, end_barrier, dtype, shape, world):
+    """csrc/allreduce.cu with `world` ranks emulated on one device: the ranks run as concurrent
+    kernels on streams of their own and exchange flags through each other's pads.  The result
+    must be oracle.rank_order_sum (fp32 sum in rank order, then one rounding), bit-identical on
+    every rank, for several calls in a row with new data on every call (monotonic flag
+    counters).  16 x 2048 needs 16 CTAs; 48 x 5504 more than 64 x 256 16-byte vectors, so the
+    grid-stride loop of its 64 CTAs runs three times.  Order-sensitive columns: (+big, +small,
+    -big) and (+big, -big, +small) on ranks 0..2 sum to 0 and to small in rank order only."""
+    m, n = shape
     numel = m * n
-    g = torch.Generator(device="cpu").manual_seed(5)
+    big, tiny = (2.0 ** 25, 1.0) if dtype == torch.bfloat16 else (32768.0, 2.0 ** -10)
+    g = torch.Generator(device="cpu").manual_seed(5 + world)
     pad_words = pk.ops.allreduce_pad_bytes() // 4
-    pads = [torch.zeros(pad_words, dtype=torch.int32, device="cuda") for _ in range(2)]
+    pads = [torch.zeros(pad_words, dtype=torch.int32, device="cuda") for _ in range(world)]
     epochs = [torch.zeros(pk.ops.allreduce_epoch_bytes() // 4, dtype=torch.int32, device="cuda")
-              for _ in range(2)]
-    bufs = [torch.empty((m, n), dtype=torch.bfloat16, device="cuda") for _ in range(2)]
-    outs = [torch.empty((m, n), dtype=torch.bfloat16, device="cuda") for _ in range(2)]
-    streams = [torch.cuda.Stream(), torch.cuda.Stream()]
+              for _ in range(world)]
+    bufs = [torch.empty((m, n), dtype=dtype, device="cuda") for _ in range(world)]
+    outs = [torch.empty((m, n), dtype=dtype, device="cuda") for _ in range(world)]
+    streams = [torch.cuda.Stream() for _ in range(world)]
     torch.cuda.synchronize()
     for it in range(4):
-        vals = [torch.randn((m, n), generator=g).to(torch.bfloat16) for _ in range(2)]
-        for r in range(2):
+        vals = [(torch.randn((m, n), generator=g) * 100).to(dtype) for _ in range(world)]
+        if world >= 3:
+            for r in range(world):  # ranks 3.. add zeros there
+                vals[r][:, 7 + it] = vals[r][:, n - 3 - it] = 0
+            for r, (x, y) in enumerate(((big, big), (tiny, -big), (-big, tiny))):
+                vals[r][:, 7 + it] = x
+                vals[r][:, n - 3 - it] = y
+        for r in range(world):
             bufs[r].copy_(vals[r])
         torch.cuda.synchronize()
-        for r in range(2):
+        for r in range(world):
             with torch.cuda.stream(streams[r]):
                 pk.ops.allreduce_oneshot(outs[r], [b.data_ptr() for b in bufs],
                                          [p.data_ptr() for p in pads], epochs[r], r, numel,
                                          end_barrier)
         torch.cuda.synchronize()
-        want = (vals[0].float() + vals[1].float()).to(torch.bfloat16)
-        assert torch.equal(outs[0].cpu(), want) and torch.equal(outs[1].cpu(), want), it
-    assert int(epochs[0][0]) == 4 and int(epochs[1][0]) == 4
+        want = orc.rank_order_sum(vals, dtype)
+        if world >= 3:
+            assert bool((want[:, 7 + it].float() == 0).all()) and bool((want[:, n - 3 - it].float() == tiny).all())
+        for r in range(world):
+            assert torch.equal(outs[r].cpu().view(torch.int16), want.view(torch.int16)), (it, r)
+    for r in range(world):
+        assert int(pk.ops.allreduce_status(epochs[r])) == 0
+        assert int(epochs[r][0]) == 4
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
-def test_peer_allreduce_two_gpus(pk):
-    """World-2 torchrun: PeerAllReduce (own kernel over symmetric memory) equals
-    ncclAllReduce on a row-parallel NVFP4 layer."""
+TP_RUNS = [(world, two_shot) for world in (2, 4, 8) for two_shot in (None, "0", "1")]
+
+
+@pytest.mark.parametrize("world,two_shot", TP_RUNS, ids=[f"{w}-{t or 'unset'}" for w, t in TP_RUNS])
+def test_peer_allreduce_two_gpus(pk, world, two_shot):
+    """torchrun over `world` GPUs with PETIT_AR_TWO_SHOT unset / 0 / 1: PeerAllReduce (own kernel
+    over symmetric memory) equals ncclAllReduce on a row-parallel NVFP4 layer, and the fused
+    GEMM + all-reduce is bit-exact on exact cases in all three formats."""
+    if torch.cuda.device_count() < world:
+        pytest.skip(f"needs {world} GPUs")
+    env = {k: v for k, v in os.environ.items() if k != "PETIT_AR_TWO_SHOT"}
+    if two_shot is not None:
+        env["PETIT_AR_TWO_SHOT"] = two_shot
     script = os.path.join(ROOT, "tests", "tp_peer_allreduce_check.py")
+    port = 29541 + TP_RUNS.index((world, two_shot))
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1",
-                        "--nproc-per-node", "2", "--master-addr", "127.0.0.1", "--master-port",
-                        "29541", script], capture_output=True, text=True, timeout=240)
+                        "--nproc-per-node", str(world), "--master-addr", "127.0.0.1", "--master-port",
+                        str(port), script], env=env, capture_output=True, text=True, timeout=600)
     assert r.returncode == 0 and "PEER_ALLREDUCE_OK" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
 
 

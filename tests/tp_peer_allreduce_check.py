@@ -10,12 +10,14 @@ import os
 import sys
 import time
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "petit-kernel_b200"))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import petit_kernel as pk  # noqa: E402
 import petit_tp  # noqa: E402
@@ -53,42 +55,43 @@ def gemm_case(rank, world):
     assert par.status() == 0
 
 
-def fused_case(rank, world, iters):
-    """petit_tp.FusedAllReduce (GEMM + all-reduce in one kernel) against the GEMM followed by
-    ncclAllReduce, on shapes where tiles are whole and where stream-K splits them, for several
-    token counts, `iters` calls each (the epoch / buffer-parity protocol has to hold)."""
+FUSED_FORMATS = (("nvfp4", torch.bfloat16), ("nvfp4", torch.float16), ("mxfp4", torch.bfloat16))
+
+
+def fused_case(rank, world, calls):
+    """petit_tp.FusedAllReduce (GEMM + all-reduce in one kernel) on exact cases
+    (oracle.make_exact_case, K split over the ranks), NVFP4 x bf16 / fp16 and MXFP4 x bf16, on
+    shapes where tiles are whole and where stream-K splits them: `calls` calls per shape with
+    inputs that change on every call, each output bit for bit oracle.rank_order_sum of the
+    ranks' exact partials (the epoch / buffer-parity protocol has to hold)."""
+    from test_gemm_exact import assert_bits
+
     far = petit_tp.FusedAllReduce()
+    dev = torch.device("cuda", torch.cuda.current_device())
     checked = []
-    for (m, n, k) in ((16, 1024, 2048 * world), (1, 8192, 1024 * world), (33, 2048, 512 * world),
-                      (64, 8192, 256 * world), (16, 8192, 3584 * world)):
-        a, q, s, gs = orc.make_nvfp4_case(m, n, k, 99 + m)
-        qs, ss = petit_tp.row_shard(q, s, world, rank)
-        a_s = petit_tp.row_shard_activation(a, world, rank).cuda()
-        ks = k // world
-        b = pk.repack_nvfp4(qs.cuda().contiguous().view(torch.int32), n, ks)
-        sp = pk.process_nvfp4_scales(ss.cuda().contiguous(), n, ks)
-        gsc = gs.cuda()
-        ref = pk.mul_nvfp4_a16(a_s, b, sp, gsc, m, n, ks, -1)
-        dist.all_reduce(ref)
-        bad = torch.zeros((), dtype=torch.int32, device="cuda")
-        first = None
-        for it in range(iters):
-            got = far.matmul(a_s, b, sp, gsc, n, ks)
-            if first is None:
-                first = got.clone()
-            bad += (got != first).any().to(torch.int32)
-        torch.cuda.synchronize()
-        assert bad.item() == 0, (m, n, k, "not reproducible across calls")
-        err = (first.float() - ref.float()).abs().max().item()
-        scale = ref.float().abs().max().item()
-        assert err <= scale * 2 ** -6, (m, n, k, err, scale)
-        gathered = [torch.empty_like(first) for _ in range(world)]
-        dist.all_gather(gathered, first)
-        assert all(torch.equal(gathered[0], x) for x in gathered), (m, n, k, "ranks differ")
-        if k <= 8192:
-            full = orc.nvfp4_gemm_ref_torch(a, q, s, gs)
-            assert orc.max_rel_err(first.float().cpu(), full) <= 1e-2
-        checked.append([m, n, k])
+    for fmt, dt in FUSED_FORMATS:
+        # (m, n, k per rank)
+        for m, n, ks in ((16, 1024, 2048), (1, 8192, 1024), (33, 2048, 512), (64, 8192, 256), (16, 2048, 3584)):
+            k = ks * world
+            a, q, s, gs, w, _ = orc.make_exact_case(fmt, dt, m * calls, n, k, 99 + m)
+            qs, ss = petit_tp.row_shard(q, s, world, rank)
+            a_s = petit_tp.row_shard_activation(a, world, rank).to(dev)  # every call's rows, staged
+            qw = qs.to(dev).contiguous().view(torch.int32)
+            if fmt == "nvfp4":
+                b, sp = pk.repack_nvfp4(qw, n, ks), pk.process_nvfp4_scales(ss.to(dev).contiguous(), n, ks)
+            else:
+                b, sp = pk.repack_mxfp4(qw, n, ks), pk.process_mxfp4_scales(ss.to(dev).contiguous(), n, ks)
+            gsc = gs.to(dev)
+            torch.cuda.synchronize()
+            outs = [far.matmul(a_s[i * m:(i + 1) * m], b, sp, gsc, n, ks, fmt) for i in range(calls)]
+            torch.cuda.synchronize()
+            a_dev = a.to(dev)
+            parts = [orc.exact_ref(a_dev[:, r * ks:(r + 1) * ks], np.ascontiguousarray(w[:, r * ks:(r + 1) * ks]),
+                                   gs.item(), dt) for r in range(world)]
+            want = orc.rank_order_sum(parts, dt)
+            for i in range(calls):
+                assert_bits(outs[i], want[i * m:(i + 1) * m], f"rank {rank} {fmt} {dt} m={m} n={n} k={k} call {i}")
+            checked.append([fmt, str(dt), m, n, k])
     assert far.status() == 0
     return checked
 
@@ -126,7 +129,8 @@ def main():
     iters = int(sys.argv[1]) if len(sys.argv) > 1 else 300
     gemm_case(rank, world)
     res = {"world": world, "iters": iters, "modes": []}
-    res["fused_gemm_allreduce"] = {"shapes": fused_case(rank, world, max(50, iters // 20)), "ok": True}
+    res["fused_gemm_allreduce"] = {"shapes": fused_case(rank, world, 6), "ok": True,
+                                   "two_shot_env": os.environ.get("PETIT_AR_TWO_SHOT")}
     for end_barrier in (False, True):
         for fenced in (False, True):
             secs = stress(rank, world, iters, end_barrier, fenced)
