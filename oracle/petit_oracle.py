@@ -422,6 +422,7 @@ def elementwise_ok(c: torch.Tensor, a: torch.Tensor, w, gs: float, dtype, bias=N
 # stream-K plan (restates launch_variant / launch_mode / Cfg of csrc/fp4_gemm.cu)
 # --------------------------------------------------------------------------
 TILE_N, TILE_K, MAX_GRID = 128, 256, 160
+MAX_GROUP_TILES = 96  # kMaxGroupTiles (csrc/fp4_gemm.h)
 MODES = ("nv_bf16", "nv_f16", "nv_f16n", "mx_bf16")
 
 
@@ -446,8 +447,9 @@ def ring_fit(mode: str, ntok: int) -> int:
 
 def stream_k_plan(m: int, n: int, k: int, ntok: int, num_sms: int, pdl: bool, cluster: bool,
                   cuts_fn, mode: str = "nv_bf16", whole_tiles_rule: bool = True,
-                  tilt_units: int = -1, tilt_late: int = -1, all_reduce: bool = False):
-    """Grid, range cuts and per-tile reducer facts of one (non-grouped) launch.
+                  tilt_units: int = -1, tilt_late: int = -1, all_reduce: bool = False,
+                  tile_rows=None, tile_groups=None):
+    """Grid, range cuts and per-tile reducer facts of one launch.
 
     cuts_fn(units, k_tiles, grid, lat, late) -> grid + 1 cuts: the library's
     petit_debug_stream_k_cuts (lat = late = 0 gives the equal split).  `cluster` is the
@@ -459,13 +461,21 @@ def stream_k_plan(m: int, n: int, k: int, ntok: int, num_sms: int, pdl: bool, cl
 
     all_reduce: the GEMM fused with its all-reduce (launch_mode with ar_world > 1, i.e.
     launch_variant<..., CL = false, AR = true>): decode tiles only (ntok 16 / 32 / 64, m <= 64),
-    never a cluster, and no arrival term in the cut tilt (late = 0)."""
+    never a cluster, and no arrival term in the cut tilt (late = 0).
+
+    tile_rows: the grouped launch (launch_variant<..., GR = true>, decode tiles only): token tile
+    t covers tile_rows[t] rows (the `rows` of group_table's entry t) instead of the rows of a
+    plain [m, k] tensor, and m_tiles = len(tile_rows).  tile_groups[t] is entry t's expert; it
+    only feeds the grouped coverage labels of plan_paths."""
     if all_reduce:
         assert ntok in (16, 32, 64) and 1 <= m <= 64, (ntok, m)
         cluster = False
+    if tile_rows is not None:
+        assert ntok in (16, 32, 64) and 1 <= len(tile_rows) <= MAX_GROUP_TILES, (ntok, len(tile_rows))
+        assert all(1 <= r <= ntok for r in tile_rows) and len(tile_groups) == len(tile_rows)
     num_sms = min(num_sms, MAX_GRID)
     n_tiles = (n + TILE_N - 1) // TILE_N
-    m_tiles = (m + ntok - 1) // ntok
+    m_tiles = (m + ntok - 1) // ntok if tile_rows is None else len(tile_rows)
     k_tiles = k // TILE_K
     cl = ntok >= 128 and cluster and n_tiles % 2 == 0 and n % TILE_N == 0
     units = (n_tiles // 2 if cl else n_tiles) * m_tiles * k_tiles
@@ -503,19 +513,44 @@ def stream_k_plan(m: int, n: int, k: int, ntok: int, num_sms: int, pdl: bool, cl
         b_first, b_last = owner(t * k_tiles), owner(t * k_tiles + k_tiles - 1)
         c = b_last - b_first
         m_tile = t % m_tiles
-        m_valid = min(ntok, m - m_tile * ntok)
+        m_valid = min(ntok, m - m_tile * ntok) if tile_rows is None else tile_rows[m_tile]
         n_tile = (2 if cl else 1) * (t // m_tiles)
         rows = [min(TILE_N, n - nt * TILE_N) for nt in ((n_tile, n_tile + 1) if cl else (n_tile,))]
         path = None if c == 0 else ("ring" if 3 < c <= fit else "reg")
-        out.append(dict(tile=t, contributors=c, m_valid=m_valid, n_partial=min(rows) < TILE_N,
+        out.append(dict(tile=t, m_tile=m_tile, contributors=c, m_valid=m_valid, n_partial=min(rows) < TILE_N,
                         path=path, l2_tail=c > 0 and path == "reg" and m_valid > 16 and c > fit))
+    # experts whose units each CTA's range holds (grouped launch)
+    cta_groups = None if tile_groups is None else [
+        {tile_groups[t % m_tiles] for t in range(cuts[b] // k_tiles, (cuts[b + 1] - 1) // k_tiles + 1)}
+        for b in range(sched_grid)]
     return dict(ntok=ntok, grid=grid, sched_grid=sched_grid, cluster=cl, whole_tiles=whole, tilt=tilt, lat=lat,
-                late=late, units=units, k_tiles=k_tiles, ring_fit=fit, cuts=cuts, tiles=out)
+                late=late, units=units, k_tiles=k_tiles, m_tiles=m_tiles, ring_fit=fit, cuts=cuts, tiles=out,
+                tile_groups=tile_groups, cta_groups=cta_groups)
 
 
 def plan_paths(plan) -> set:
-    """Coverage labels of one launch (see stream_k_plan)."""
+    """Coverage labels of one launch (see stream_k_plan).  A grouped launch adds:
+      group_switch      a CTA's range holds units of two or more experts (weights, scales and gs
+                        change inside one CTA's k-range);
+      split_group_tail  a split tile with fewer than ntok rows that is not the last token tile
+                        (the rows its token tile loads after its last row are the next expert's);
+      direct_store      a tile whose rows are not a multiple of 16 (its last 16-token group is
+                        written with 16-byte stores instead of a TMA box);
+      multi_tile_group  an expert with more than one token tile;
+      table_full        a table of exactly MAX_GROUP_TILES entries."""
     got = set()
+    if plan["tile_groups"] is not None:
+        if any(len(g) >= 2 for g in plan["cta_groups"]):
+            got.add("group_switch")
+        for t in plan["tiles"]:
+            if t["contributors"] and t["m_valid"] < plan["ntok"] and t["m_tile"] != plan["m_tiles"] - 1:
+                got.add("split_group_tail")
+            if t["m_valid"] % 16:
+                got.add("direct_store")
+        if len(set(plan["tile_groups"])) < plan["m_tiles"]:
+            got.add("multi_tile_group")
+        if plan["m_tiles"] == MAX_GROUP_TILES:
+            got.add("table_full")
     if plan["whole_tiles"]:
         got.add("whole_tiles")
     if plan["ntok"] >= 128:
@@ -537,6 +572,46 @@ def plan_paths(plan) -> set:
         if t["m_valid"] < plan["ntok"]:
             got.add("split_partial_m")
     return got
+
+
+# --------------------------------------------------------------------------
+# grouped (MoE) launch (restates petit_gemm_fp4_a16_grouped of csrc/capi.cu)
+# --------------------------------------------------------------------------
+def group_table(counts, ntok: int):
+    """[(group, row0, rows)]: the token tiles of the single grouped launch.  Expert g owns rows
+    [sum(counts[:g]), sum(counts[:g + 1])) of the concatenated activations / output; each of its
+    ntok-row blocks is one entry, the last one holding the remainder; empty experts have none."""
+    out, row = [], 0
+    for g, c in enumerate(counts):
+        for r in range(0, c, ntok):
+            out.append((g, row + r, min(ntok, c - r)))
+        row += c
+    return out
+
+
+def grouped_launch(counts, n: int, k: int, sid: int, dtype, contiguous: bool = True, bias: bool = False,
+                   single_env: bool = True):
+    """How petit_gemm_fp4_a16_grouped issues a call: ("single", ntok, group_table(counts, ntok))
+    or ("one_by_one", None, [(group, m)] of the live groups in order).  One launch needs all of:
+    PETIT_GROUPED_SINGLE not 0 (single_env), no bias, n and k non-zero, the live groups'
+    activations and outputs consecutive row blocks of one tensor (contiguous), at least two live
+    groups, a decode tile (sid -1: 16 / 32 / 64 tokens by the largest group; an explicit id must
+    name a tile of <= 64 tokens) and a table of at most MAX_GROUP_TILES entries.  dtype is the
+    activation type (bf16 or fp16: both have the single form)."""
+    assert _torch_dtype(dtype) in (torch.bfloat16, torch.float16)
+    live = [(g, c) for g, c in enumerate(counts) if c]
+    ntok = 0
+    if single_env and not bias and n and k and contiguous and len(live) >= 2:
+        if sid == -1:
+            top = max(c for _, c in live)
+            ntok = 16 if top <= 16 else (32 if top <= 32 else 64)
+        elif (sid & 0xFF) * 16 <= 64:
+            ntok = (sid & 0xFF) * 16
+    if ntok:
+        table = group_table(counts, ntok)
+        if len(table) <= MAX_GROUP_TILES:
+            return "single", ntok, table
+    return "one_by_one", None, live
 
 
 def rank_order_sum(partials, dtype) -> torch.Tensor:

@@ -289,3 +289,143 @@ def test_fused_allreduce_cases_fit_and_cover_every_path(cuts_fn, mode):
     rems = {n % 128 for _, _, n, _, _ in tfa.sequence_cases(petit_kernel, mode)}
     assert rems == ({32, 96} if mode in ("mx_bf16", "nv_f16n") else {16, 112})
     assert all(x != y for x, y in zip(tfa.SEQ_M, tfa.SEQ_M[1:])) and set(tfa.SEQ_M) == {1, 5, 16, 17, 33, 48, 64}
+
+
+# ------------------------------------------------------------------ grouped (MoE) launch
+def _ids():
+    """Solution ids of NVFP4 x bf16 by token tile (the id layout of capi.cu make_solution)."""
+    import petit_kernel
+
+    return {tge.solution_ntok(petit_kernel, "nv_bf16", 16, 1024, 2048, s): s
+            for s in tge.solutions(petit_kernel, "nv_bf16", 16, 1024, 2048) if s != -1}
+
+
+def test_group_table_and_grouped_launch_follow_the_rules():
+    """group_table / grouped_launch against hand-worked routings: empty groups at the front, in
+    the middle and at the end, one live group, all groups empty, 96 and 97 tiles, explicit ids
+    of every token tile, a bias, PETIT_GROUPED_SINGLE=0 and groups in separate tensors."""
+    ids = _ids()
+    assert sorted(ids) == [16, 32, 64, 128, 256]
+    assert orc.group_table([0, 5, 0, 33, 1, 0], 16) == [(1, 0, 5), (3, 5, 16), (3, 21, 16), (3, 37, 1), (4, 38, 1)]
+    assert orc.group_table([0, 5, 0, 33, 1, 0], 64) == [(1, 0, 5), (3, 5, 33), (4, 38, 1)]
+    assert orc.group_table([0, 0], 16) == []
+    n, k, dt = 1024, 2048, torch.bfloat16
+    single = lambda c, sid=-1, **kw: orc.grouped_launch(c, n, k, sid, dt, **kw)  # noqa: E731
+    # -1: the token tile follows the largest group
+    for top, ntok in ((1, 16), (16, 16), (17, 32), (32, 32), (33, 64), (64, 64), (65, 64), (500, 64)):
+        form, got, table = single([0, 3, 0, top, 0])
+        assert (form, got) == ("single", ntok) and table == orc.group_table([0, 3, 0, top, 0], ntok)
+    # explicit ids: decode tiles make one launch, 128 / 256 go one by one
+    for t in (16, 32, 64):
+        assert single([9, 0, 40], ids[t])[:2] == ("single", t)
+    for t in (128, 256):
+        assert single([9, 0, 40], ids[t]) == ("one_by_one", None, [(0, 9), (2, 40)])
+    # one live group, no live group, a bias, the switch, separate tensors: one by one
+    assert single([0, 0, 7, 0]) == ("one_by_one", None, [(2, 7)])
+    assert single([0, 0, 0]) == ("one_by_one", None, [])
+    assert single([3, 4], bias=True) == ("one_by_one", None, [(0, 3), (1, 4)])
+    assert single([3, 4], single_env=False)[0] == single([3, 4], contiguous=False)[0] == "one_by_one"
+    assert orc.grouped_launch([3, 4], n, k, -1, torch.float16)[:2] == ("single", 16)
+    # the table holds 96 entries, not 97
+    assert len(single([1] * 96)[2]) == 96 and single([1] * 97)[0] == "one_by_one"
+    assert len(single([16] * 96)[2]) == 96 and single([16] * 95 + [17], ids[16])[0] == "one_by_one"
+    assert single([16] * 95 + [17])[:2] == ("single", 32)
+    assert single([33] * 49, ids[32])[0] == "one_by_one" and len(single([33] * 49, ids[64])[2]) == 49
+    assert len(single([32] * 47 + [17], ids[16])[2]) == 96 and single([32] * 47 + [33], ids[16])[0] == "one_by_one"
+
+
+def test_grouped_launch_on_random_routings():
+    """Random routings (top-k of random token counts over up to 160 experts): the single form's
+    table covers every token once, in order, in tiles of at most ntok rows that never straddle two
+    experts; a routing takes the single form exactly when it has two live groups and a table of
+    at most 96 entries."""
+    rs = np.random.RandomState(0)
+    for it in range(300):
+        e = int(rs.randint(1, 161))
+        counts = [int(c) for c in rs.poisson(rs.choice([0.3, 2.0, 12.0, 60.0]), size=e) * (rs.rand(e) < 0.7)]
+        form, ntok, table = orc.grouped_launch(counts, 1024, 2048, -1, torch.bfloat16)
+        live = [g for g, c in enumerate(counts) if c]
+        if form == "one_by_one":
+            assert table == [(g, counts[g]) for g in live]
+            top = max(counts) if live else 0
+            t = 16 if top <= 16 else 32 if top <= 32 else 64
+            assert len(live) < 2 or len(orc.group_table(counts, t)) > orc.MAX_GROUP_TILES
+            continue
+        assert len(live) >= 2 and len(table) <= orc.MAX_GROUP_TILES and ntok >= max(counts) or ntok == 64
+        off = np.concatenate([[0], np.cumsum(counts)])
+        row = 0
+        for g, row0, rows in table:
+            assert row0 == row and 1 <= rows <= ntok and off[g] <= row0 and row0 + rows <= off[g + 1]
+            row += rows
+        assert row == sum(counts)
+
+
+def test_grouped_plan_equals_the_plain_plan_for_one_group(cuts_fn):
+    """stream_k_plan's tile_rows input changes nothing but m_tiles and m_valid: the table of one
+    group of m tokens is the plain launch's token tiles, so the plans agree."""
+    for m, n, k, ntok in ((48, 4096, 4096, 16), (64, 128, 28672, 64), (17, 1040, 4096, 32), (16, 8192, 1024, 16)):
+        table = orc.group_table([m], ntok)
+        plain = orc.stream_k_plan(m, n, k, ntok, 148, True, True, cuts_fn)
+        grp = orc.stream_k_plan(m, n, k, ntok, 148, True, True, cuts_fn, tile_rows=[r for _, _, r in table],
+                                tile_groups=[g for g, _, _ in table])
+        for key in ("grid", "cuts", "whole_tiles", "tilt", "tiles"):
+            assert plain[key] == grp[key], (m, n, k, key)
+        assert orc.plan_paths(plain) <= orc.plan_paths(grp)
+        assert "group_switch" not in orc.plan_paths(grp) and "multi_tile_group" in orc.plan_paths(grp) or m <= ntok
+
+
+def test_grouped_exact_ref_rejects_planted_defects():
+    """Per-expert exact_ref against outputs a subtly wrong grouped kernel would write: the
+    neighbour expert's weights for one tile, the neighbour's gs for one expert, one row computed
+    as a row of the next group, and a 16-row box written past a group's end (the next expert's
+    first rows multiplied with this expert's weights).  Bit equality and elementwise_ok reject all
+    four; the 1e-2 normwise bar accepts the neighbour's gs."""
+    import test_grouped_exact as tg
+
+    dt = torch.bfloat16
+    n, k, counts = 256, 1024, [5, 7, 3, 9]
+    cases = [orc.make_exact_case("nvfp4", dt, c, n, k, 40 + g) for g, c in enumerate(counts)]
+    gs = [tg.expert_gs(g) for g in range(len(counts))]
+    off = tg.offsets_of(counts)
+    ref = lambda a, g, gsv=None: orc.exact_ref(a, cases[g][4], gs[g] if gsv is None else gsv, dt)  # noqa: E731
+    want = torch.cat([ref(c[0], g) for g, c in enumerate(cases)])
+    a_all = torch.cat([c[0] for c in cases])
+    f64 = torch.cat([(c[0].double() @ torch.from_numpy(c[4]).double().t()) * gs[g] for g, c in enumerate(cases)])
+    defects = {}
+    d = want.clone()
+    d[off[1]:off[2], :128] = ref(cases[1][0], 2)[:, :128]          # expert 1, n-tile 0: expert 2's weights
+    defects["neighbour_weights"] = d
+    d = want.clone()
+    d[off[2]:off[3]] = ref(cases[2][0], 2, gs[3])                   # expert 2 scaled by expert 3's gs
+    defects["neighbour_gs"] = d
+    d = want.clone()
+    d[off[1] - 1] = ref(cases[0][0][-1:], 1)[0]                     # expert 0's last row as expert 1's
+    defects["row_shifted"] = d
+    d = want.clone()
+    d[off[1]:off[0] + 16] = ref(a_all[off[1]:off[0] + 16], 0)       # expert 0's 16-row box over expert 1
+    defects["box_past_end"] = d
+    old_bar = {}
+    for name, c in defects.items():
+        assert not orc.bits_equal_pm0(c, want), name
+        ok = all(orc.elementwise_ok(c[off[g]:off[g + 1]], cases[g][0], cases[g][4], gs[g], dt)
+                 for g in range(len(counts)))
+        assert not ok, name
+        old_bar[name] = orc.max_rel_err(c, f64) <= 1e-2
+    assert old_bar == {"neighbour_weights": False, "neighbour_gs": True, "row_shifted": False, "box_past_end": False}
+
+
+@pytest.mark.parametrize("mode", list(tge.MODES))
+def test_grouped_routings_cover_every_path(cuts_fn, mode):
+    """The grouped GPU file's coverage assertion at the B200's 148 SMs, and the launch forms its
+    routings are meant to take."""
+    import petit_kernel
+    import test_grouped_exact as tg
+
+    table = tg.grouped_coverage(petit_kernel, cuts_fn, mode, 148)
+    assert [lab for lab in tg.GROUPED_REQUIRED if lab not in table] == []
+    dt = tge.MODES[mode][1]
+    forms = {r: orc.grouped_launch(c, tg.mode_n(mode, n), k, -1, dt)[0] for r, (n, k, c) in tg.ROUTINGS.items()}
+    assert {r for r, f in forms.items() if f == "one_by_one"} == {"one_expert", "all_empty", "tiles_97"}
+    assert len(orc.group_table(tg.ROUTINGS["tiles_96"][2], 16)) == 96
+    assert len(orc.group_table(tg.ROUTINGS["tiles_97"][2], 16)) == 97
+    assert len(tg.QWEN3) == 128 and sum(tg.QWEN3) == 16 * 8

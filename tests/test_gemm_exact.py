@@ -406,45 +406,6 @@ def test_fused_silu_mul_on_exact_gemm(pk, mode):
             assert (got == want).float().mean().item() > 0.98
 
 
-GROUPED_CASES = ((512, 1024, [5, 0, 33, 1, 16, 70]),      # 64-token tiles
-                 (2048, 4096, [3, 1, 0, 7, 2, 16, 4, 1]),  # 16-token tiles split by stream-K
-                 (1040, 768, [17, 32, 0, 0, 9]))           # 32-token tiles, partial n-tile
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("mode", ["nv_bf16", "nv_f16", "mx_bf16"])
-def test_grouped_exact_single_launch_equals_one_by_one(pk, mode):
-    """Grouped GEMM with a distinct non-power-of-two gs per expert, ragged and empty groups,
-    NaN-filled outputs: the single-launch kernel and the one-by-one launches both equal the
-    per-expert exact reference, hence each other, bit for bit."""
-    fmt, dt, _ = MODES[mode]
-    for n, k, counts in GROUPED_CASES:
-        n = mode_shape(mode, 16, n, k)[1]
-        offsets = np.concatenate([[0], np.cumsum(counts)]).tolist()
-        a_all, bs, ss, gss, wants = [], [], [], [], []
-        for g, cnt in enumerate(counts):
-            a, q, s, _, w, _ = orc.make_exact_case(fmt, dt, max(cnt, 1), n, k, 200 + g)
-            gs = 0.7 + 0.05 * g
-            b, sp = pack(pk, mode, q, s, n, k)
-            a_all.append(a[:cnt]); bs.append(b); ss.append(sp); gss.append(gs)
-            wants.append(orc.exact_ref(a[:cnt], w, gs, dt))
-        a_cat = torch.cat(a_all).cuda().contiguous()
-        gsc = torch.tensor(gss, dtype=torch.float32, device="cuda")
-        outs = []
-        for single in ("1", "0"):
-            os.environ["PETIT_GROUPED_SINGLE"] = single
-            try:
-                out = torch.full((offsets[-1], n), float("nan"), dtype=dt, device="cuda")
-                pk.ops.mul_fp4_a16_grouped_out(out, a_cat, torch.stack(bs), torch.stack(ss), gsc, offsets,
-                                               n, k, -1, fmt == "mxfp4")
-                torch.cuda.synchronize()
-            finally:
-                os.environ.pop("PETIT_GROUPED_SINGLE", None)
-            outs.append(out.cpu())
-            assert_bits(out, torch.cat(wants), f"{mode} grouped n={n} k={k} single={single}")
-        assert torch.equal(outs[0].view(torch.int16), outs[1].view(torch.int16))
-
-
 # ------------------------------------------------------------------ launch configuration
 # (mode, m, n, k): computed in this process and again in subprocesses with PETIT_PDL=0,
 # PETIT_CLUSTER=0, PETIT_WHOLE_TILES=0 and other tilt parameters
